@@ -253,6 +253,40 @@ def ref_cuda_leg(s, stepsize, grad_out, out, grads, chunk=16, reps=7, warm=2):
 
 
 # ----------------------------------------------------------------------------------------------------------------
+# --dump-outputs: the outputs of the timed path, so that two builds can be compared output for output
+# ----------------------------------------------------------------------------------------------------------------
+DUMP_BYTES = 62_000_000        # all arrays together; with the .npy headers the files stay under 64 MB
+
+
+def sample_outputs(arrays, budget=DUMP_BYTES, seed=1112):
+    """Host float32 copies of the device tensors `arrays` (name -> tensor) within `budget` bytes.  Arrays are taken in order of
+    size, each whole if it fits its share of what is left, otherwise as a fixed, seeded sample of its rows (the last axis
+    kept whole: RGBA of a pixel or a voxel), sorted by row index -- the same rows in every run with the same arguments."""
+    out = {}
+    left = budget
+    names = sorted(arrays, key=lambda n: arrays[n].numel())
+    for i, name in enumerate(names):
+        x = arrays[name].detach().float()
+        share = left // (len(names) - i)
+        if x.numel() * 4 > share:
+            rows = x.reshape(-1, x.shape[-1])
+            g = torch.Generator().manual_seed(seed + i)
+            idx = torch.randint(rows.shape[0], (share // (rows.shape[1] * 4),), generator=g).unique()
+            x = rows[idx.to(rows.device)]
+        out[name] = x.cpu().numpy()
+        left -= out[name].nbytes
+    return out
+
+
+def write_outputs(outdir, arrays):
+    import numpy as np
+    os.makedirs(outdir, exist_ok=True)
+    for name, a in arrays.items():
+        np.save(os.path.join(outdir, name + ".npy"), a)
+    log("outputs of the last timed step written to %s (%s)" % (outdir, ", ".join("%s %s" % (n, list(a.shape)) for n, a in arrays.items())))
+
+
+# ----------------------------------------------------------------------------------------------------------------
 # our arm
 # ----------------------------------------------------------------------------------------------------------------
 def run_ours(args, rank, world):
@@ -286,16 +320,16 @@ def run_ours(args, rank, world):
         torch.cuda.synchronize()
 
     def step():
+        """Returns the images and the flat buffer the subject's (all-reduced) primitive gradients go to."""
         for x in leaves:
             x.grad = None
         out = mvpraymarch(s["raypos"], s["raydir"], stepsize, s["tminmax"], (leaves[0], leaves[1], leaves[2]), leaves[3], None)
         out.backward(grad_out)
         # views of a step share the subject's primitives: local sum over the rank's views, one all-reduce (SURVEY 8e)
-        red.reduce(leaves[3].grad, leaves[0].grad, leaves[1].grad, leaves[2].grad)
-        return out
+        return out, red.reduce(leaves[3].grad, leaves[0].grad, leaves[1].grad, leaves[2].grad)
 
     for i in range(args.warmup):
-        out = step()
+        out, _ = step()
         red.finish()
         torch.cuda.synchronize()
         log("warmup step %d done" % i)
@@ -307,11 +341,17 @@ def run_ours(args, rank, world):
     barrier()
     e0.record()
     for _ in range(args.steps):
-        out = step()
+        out, out_flat = step()
     red.finish()                 # the compute stream waits for the last all-reduce: it is inside the timed region
     e1.record()
     barrier()
     ms = e0.elapsed_time(e1)
+    dump = None
+    if args.dump_outputs and rank == 0:
+        # what the caller of the timed path receives from its last step: rank 0's images and the subject's reduced gradients
+        g_tpl, g_pos, g_rot, g_scale = red.views(out_flat, k, t, t, t)
+        dump = sample_outputs({"rayrgba": out.detach(), "grad_template": g_tpl, "grad_primpos": g_pos,
+                               "grad_primrot": g_rot, "grad_primscale": g_scale})
     # the collective alone (not overlapped), for the record
     allreduce_ms = None
     if world > 1:
@@ -327,6 +367,8 @@ def run_ours(args, rank, world):
         allreduce_ms = float(ta.item())
     log("timed region: %.1f ms for %d steps" % (ms, args.steps))
     clocks = sampler.stop() if rank == 0 else None
+    if dump is not None:
+        write_outputs(args.dump_outputs, dump)
     tms = torch.tensor([ms], device=dev)
     if world > 1:
         dist.all_reduce(tms, op=dist.ReduceOp.MAX)
@@ -473,7 +515,7 @@ def run_ours(args, rank, world):
                       "image_max_rel_diff_vs_host_formula_rays": cam_img_diff,
                       "kernel_ms": {"forward_all_views_per_rank": fwd_cam_ms, "backward_all_views_per_rank": bwd_cam_ms}}
         del o_cam
-        out = step()                 # the leaves' gradients are those of the headline configuration again (the parity leg reads them)
+        out, _ = step()              # the leaves' gradients are those of the headline configuration again (the parity leg reads them)
         red.finish()
         torch.cuda.synchronize()
         log("camera-ray configuration: %.2f ms per step (kernels %.2f + %.2f)" % (camera_cfg["ms_per_step"], fwd_cam_ms, bwd_cam_ms))
@@ -705,7 +747,11 @@ def main():
     ap.add_argument("--no-cpu-baseline", action="store_true")
     ap.add_argument("--no-shared-leg", action="store_true", help="skip the shared-primitive ([1,K,...]) configuration")
     ap.add_argument("--no-check", action="store_true", help="skip the reference-CUDA legs (ref_cuda_baseline, parity_check)")
+    ap.add_argument("--dump-outputs", metavar="DIR", help="write the images and reduced gradients of the last timed step to "
+                    "DIR/<name>.npy (float32; a fixed, seeded sample of the larger arrays, at most 64 MB in all)")
     args = ap.parse_args()
+    if args.steps < 1:
+        ap.error("--steps must be at least 1")
     args.warmup = max(args.warmup, 0)
     rank = int(os.environ.get("RANK", 0))
     world = int(os.environ.get("WORLD_SIZE", 1))

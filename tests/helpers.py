@@ -120,6 +120,83 @@ def build_case(name):
     return s, grad
 
 
+# ----------------------------------------------------------------------------------------------------------
+# Scenes compared with the reference CUDA extension at sizes whose outputs are too large to store whole: a seeded sample
+# of each reference output is kept in tests/golden/sampled_<name>.npz (tests/golden/make_sampled_golden.py)
+# ----------------------------------------------------------------------------------------------------------
+def _gpu_scene(n_views, H, W, K, T, alpha_mu, alpha_sigma, grad_seed, view_offset=0):
+    from ava256_b200 import scene
+    s = scene.make_scene(n_views, H, W, K, T, view_offset=view_offset, alpha_mu=alpha_mu, alpha_sigma=alpha_sigma, device="cuda")
+    grad = torch.randn(n_views, H, W, 4, device="cuda", generator=torch.Generator(device="cuda").manual_seed(grad_seed))
+    return s, grad
+
+
+def _head_256x168():
+    from ava256_b200 import scene
+    s = scene.make_scene(2, 256, 168, 1024, 8, alpha_mu=3.0, alpha_sigma=3.0, share_primitives=False)
+    return s, torch.randn(2, 256, 168, 4, generator=torch.Generator().manual_seed(99))
+
+
+SAMPLED_CASES = {
+    # BASELINE.json config 2: 1 subject, 4 views 512x334, K=4096, 16^3
+    "c2": lambda: _gpu_scene(4, 512, 334, 4096, 16, 17.0, 6.0, 5),
+    # the scene bench.py times (C3: 1024x667, K=16384, 8^3, alpha 17/6, dt=1/256), views 0, 1 and the two most oblique ones
+    "c3_views0": lambda: _gpu_scene(2, 1024, 667, 16384, 8, 17.0, 6.0, 6, view_offset=0),
+    "c3_views78": lambda: _gpu_scene(2, 1024, 667, 16384, 8, 17.0, 6.0, 84, view_offset=78),
+    # mid-size head scene, inputs made on the CPU
+    "head_256x168": _head_256x168,
+}
+
+
+def dome_cameras(n, H, W):
+    """(campos, camrot, focal, princpt) of `n` dome cameras, fp32 on the CPU."""
+    from ava256_b200 import scene
+    campos, camrot = scene.look_at_cameras(n)
+    ds = scene.FULLRES_H / H
+    focal = torch.full((n, 2), scene.FOCAL_FULLRES / ds)
+    princpt = torch.tensor([[W / 2.0, H / 2.0]]).expand(n, 2).contiguous()
+    return campos.float().contiguous(), camrot.float().contiguous(), focal, princpt
+
+
+def golden_sample(x, key, n=1024, seed=0):
+    """Golden entries of tensor `x`: n element indices (half uniform over x, half uniform over its nonzero elements), the
+    values there, and max|x| over the whole tensor."""
+    flat = x.detach().reshape(-1)
+    assert flat.numel() < 2 ** 31
+    g = torch.Generator().manual_seed(seed)
+    idx = torch.randint(flat.numel(), (n // 2,), generator=g)
+    nz = flat.nonzero().view(-1).cpu()
+    if nz.numel():
+        idx = torch.cat([idx, nz[torch.randint(nz.numel(), (n - n // 2,), generator=g)]])
+    idx = idx.unique()
+    return {key + "__idx": idx.numpy().astype(np.int32), key + "__val": flat[idx.to(flat.device)].cpu().numpy(),
+            key + "__absmax": np.float64(flat.abs().max().item())}
+
+
+def sampled_relerr(x, gold, key):
+    """relerr of tensor `x` against the reference tensor `key` of a golden_sample file, as far as the sample shows it: the
+    larger of max|x - ref| over the sampled elements and |max|x| - max|ref||, over max|ref| of the whole tensor.  Both are
+    lower bounds of max|x - ref| over the whole tensor, so any bound relerr(x, ref) meets holds for them too."""
+    flat = x.detach().reshape(-1)
+    idx = torch.from_numpy(gold[key + "__idx"].astype(np.int64)).to(flat.device)
+    val = torch.from_numpy(gold[key + "__val"]).to(flat.device)
+    absmax = float(gold[key + "__absmax"])
+    d = float((flat[idx].double() - val.double()).abs().max())
+    m = abs(float(flat.abs().max()) - absmax)
+    return max(d, m) / max(absmax, 1e-30)
+
+
+def golden_mask(mask, key):
+    """A boolean tensor stored whole, one bit per element."""
+    m = mask.detach().reshape(-1).cpu().numpy().astype(bool)
+    return {key + "__bits": np.packbits(m), key + "__shape": np.array(mask.shape, np.int64)}
+
+
+def load_golden_mask(gold, key):
+    shape = tuple(int(v) for v in gold[key + "__shape"])
+    return np.unpackbits(gold[key + "__bits"], count=int(np.prod(shape))).reshape(shape).astype(bool)
+
+
 EDGE_KINDS = ("zero_scale", "rays_miss_volume", "large_step", "tiny_step")
 
 

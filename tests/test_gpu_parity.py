@@ -1,8 +1,8 @@
 """GPU parity tests (run on the B200 box: `pytest -m gpu`).  Every call goes through the public op
 (extensions.mvpraymarch.mvpraymarch.mvpraymarch -> ctypes -> C-ABI); the checkers are
   (a) oracle/mvp_oracle.c on the same seeded inputs,
-  (b) the committed golden vectors produced by the unmodified reference CUDA extension (tests/golden/*.npz),
-  (c) the reference extension itself when oracle/_ref travelled to the box.
+  (b) the committed golden vectors produced by the unmodified reference CUDA extension (tests/golden/*.npz; at the
+      mid-size head scene a seeded sample of them, tests/golden/sampled_*.npz).
 Tolerances are the north star's: forward max|d|/max|ref| <= 1e-4, gradients <= 1e-3."""
 import os
 
@@ -10,7 +10,7 @@ import numpy as np
 import pytest
 import torch
 
-from tests.helpers import CASES, build_case, edge_scene, relerr, scene_args_np
+from tests.helpers import CASES, SAMPLED_CASES, build_case, edge_scene, relerr, sampled_relerr, scene_args_np
 
 pytestmark = pytest.mark.gpu
 
@@ -92,23 +92,14 @@ def test_non_pinhole_rays_fall_back():
 
 
 def test_reference_extension_side_by_side():
-    """Mid-size head scene against the reference kernels compiled for sm_100 (needs oracle/_ref on the box)."""
-    from tests import refext
-    if not refext.available():
-        pytest.skip("oracle/_ref/mvpraymarchlib.so not present")
-    from ava256_b200 import scene
-    s = scene.make_scene(2, 256, 168, 1024, 8, alpha_mu=3.0, alpha_sigma=3.0, share_primitives=False)
-    g = torch.Generator().manual_seed(99)
-    grad = torch.randn(2, 256, 168, 4, generator=g)
+    """Mid-size head scene against the reference kernels compiled for sm_100 (their outputs stored as seeded samples,
+    tests/golden/sampled_head_256x168.npz)."""
+    s, grad = SAMPLED_CASES["head_256x168"]()
     out, grads = run_ours(s, grad)
-    t = {k: (v.cuda() if torch.is_tensor(v) else v) for k, v in s.items()}
-    rgba, sat, st = refext.forward(t["raypos"], t["raydir"], t["stepsize"], t["tminmax"], t["primpos"], t["primrot"],
-                                   t["primscale"], t["template"])
-    gref = refext.backward(t["raypos"], t["raydir"], t["stepsize"], t["tminmax"], t["primpos"], t["primrot"],
-                           t["primscale"], t["template"], rgba, sat, st, grad.cuda())
-    assert relerr(out, rgba.cpu().numpy()) <= FWD_TOL
-    for nm, g_, r in zip(("primpos", "primrot", "primscale", "template"), grads, gref):
-        assert relerr(g_, r.cpu().numpy()) <= BWD_TOL, nm
+    gold = np.load(os.path.join(GOLDEN, "sampled_head_256x168.npz"))
+    assert sampled_relerr(torch.from_numpy(out), gold, "rayrgba") <= FWD_TOL
+    for nm, g_ in zip(("primpos", "primrot", "primscale", "template"), grads):
+        assert sampled_relerr(torch.from_numpy(g_), gold, "grad_" + nm) <= BWD_TOL, nm
 
 
 @pytest.mark.parametrize("kind", ["zero_scale", "rays_miss_volume", "large_step", "tiny_step"])

@@ -2,49 +2,41 @@
 (2) the stand-alone accel / ACCEL_VALID C-ABI path; (3) size-independent properties at BASELINE.json's full
 per-view sizes (C2: 512x334, K=4096, 16^3 and C3: 1024x667, K=16384, 8^3), where the CPU oracle is too slow."""
 import ctypes
+import os
 
 import numpy as np
 import pytest
 import torch
 
-from tests.helpers import relerr
+from tests.helpers import dome_cameras, relerr, sampled_relerr
 
 pytestmark = pytest.mark.gpu
 
 
-def _cams(n, H, W):
-    from ava256_b200 import scene
-    campos, camrot = scene.look_at_cameras(n)
-    ds = scene.FULLRES_H / H
-    focal = torch.full((n, 2), scene.FOCAL_FULLRES / ds)
-    princpt = torch.tensor([[W / 2.0, H / 2.0]]).expand(n, 2).contiguous()
-    return campos.float().contiguous(), camrot.float().contiguous(), focal, princpt
-
-
 @pytest.mark.parametrize("with_pixelcoords", [False, True])
 def test_compute_raydirs_matches_host_formula_and_reference(with_pixelcoords):
+    """Against the host formula and against the reference's own kernel (its outputs stored as seeded samples,
+    tests/golden/sampled_raydirs.npz)."""
     from ava256_b200 import scene
     from extensions.utils.utils import compute_raydirs
-    from tests import refext
     n, H, W = 3, 77, 53
-    campos, camrot, focal, princpt = _cams(n, H, W)
+    campos, camrot, focal, princpt = dome_cameras(n, H, W)
     d = lambda t: t.cuda()  # noqa: E731
     if with_pixelcoords:
         py, px = torch.meshgrid(torch.arange(H).float(), torch.arange(W).float(), indexing="ij")
-        pc = torch.stack([px, py], dim=-1)[None].repeat(n, 1, 1, 1).contiguous().cuda()
-        arg = pc
+        arg = torch.stack([px, py], dim=-1)[None].repeat(n, 1, 1, 1).contiguous().cuda()
     else:
-        pc, arg = None, (W, H)
+        arg = (W, H)
     rp, rd, tmm = compute_raydirs(d(campos), d(camrot), d(focal), d(princpt), arg, scene.VOLRADIUS)
     hp, hd, ht = scene.compute_raydirs_host(campos, camrot, focal, princpt, H, W)
     assert relerr(rp.cpu().numpy(), hp.numpy()) < 1e-6
     assert relerr(rd.cpu().numpy(), hd.numpy()) < 1e-6
     assert relerr(tmm.cpu().numpy(), ht.numpy()) < 1e-5
-    if refext.utils_available():
-        qp, qd, qt = refext.compute_raydirs(d(campos), d(camrot), d(focal), d(princpt), pc, H, W, scene.VOLRADIUS)
-        assert torch.equal(rp, qp)
-        assert relerr(rd.cpu().numpy(), qd.cpu().numpy()) < 2e-7
-        assert relerr(tmm.cpu().numpy(), qt.cpu().numpy()) < 1e-6
+    gold = np.load(os.path.join(os.path.dirname(os.path.abspath(__file__)), "golden", "sampled_raydirs.npz"))
+    tag = "pc1_" if with_pixelcoords else "pc0_"
+    assert np.array_equal(rp.cpu().numpy(), gold[tag + "raypos"])
+    assert sampled_relerr(rd, gold, tag + "raydir") < 2e-7
+    assert sampled_relerr(tmm, gold, tag + "tminmax") < 1e-6
 
 
 def test_generated_rays_render_like_host_rays():
@@ -54,7 +46,7 @@ def test_generated_rays_render_like_host_rays():
     from extensions.utils.utils import compute_raydirs
     from oracle import oracle
     n, H, W, K, T = 1, 48, 32, 64, 8
-    campos, camrot, focal, princpt = _cams(n, H, W)
+    campos, camrot, focal, princpt = dome_cameras(n, H, W)
     rp, rd, tmm = compute_raydirs(campos.cuda(), camrot.cuda(), focal.cuda(), princpt.cuda(), (W, H), scene.VOLRADIUS)
     s = scene.make_scene(n, H, W, K, T, alpha_mu=2.0, alpha_sigma=2.0)
     with torch.no_grad():
