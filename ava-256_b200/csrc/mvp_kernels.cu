@@ -1014,14 +1014,14 @@ struct Params {
     float dt, fadescale, fadeexp;
     const float *raypos, *raydir, *tminmax;
     const float4 *raycam;         // per view 4 x float4 (raygen.h): the rays are generated from it instead of read (mvp_camera); or NULL
-    const float *tplate;
+    const float *tplate;          // voxels of the kernels' TP: float4, or four bf16 (MVP_FLAG_TPLATE_BF16)
     const float4 *pack;
     const unsigned *rx, *ry;
     const int *rowcnt;
     const RowEntry *rowlist;
     int R, rowcap;
     int TXn, TYn;
-    unsigned slab_bytes;          // TD*TH*TW*16
+    unsigned slab_bytes;          // TD*TH*TW*sizeof(voxel): 16 (fp32 payload) or 8 (bf16)
     const int *order, *rankof;    // explicit marching order (per view [K]) and its inverse, or NULL: the fixed-order rotation
     long long *tileclk;           // MVP_TILE_CLOCKS diagnostics
     int CXn, CYn;                 // CTAs (kBlkTX x kBlkTY tiles) per view in x / y
@@ -1089,7 +1089,7 @@ __device__ __forceinline__ bool tile_bucket_empty(const Params &p, int n, int tx
 // the first-hit depths (0.57 vs 0.70 ms per 1024x667 view) because neighbouring slabs sit at randomly different
 // depths while the sweep planes stay coherent.
 // Returns false when the list would exceed CAP (< 512): the caller hands the tile to the 512-entry kernel.
-template <int CAP, bool kPrefetch>
+template <int CAP, bool kPrefetch, typename TP>
 __device__ __forceinline__ bool build_tile_list(const Params &p, float rdt, int n, int tx, int ty, int lane, TileCtx &c,
                                                 int *s_k, int *s_iv, RowEntry *s_stage, unsigned long long *s_bar, float &t,
                                                 float &x, float &y, float &z, float &r1e, int &j0) {
@@ -1236,7 +1236,14 @@ __device__ __forceinline__ bool build_tile_list(const Params &p, float rdt, int 
         const char *tp = reinterpret_cast<const char *>(p.tplate) + (size_t)(n * p.pview) * p.K * p.slab_bytes;
         for (int i = lane; i < nl; i += 32) {
             const char *a = tp + (size_t)s_k[i] * p.slab_bytes;
-            asm volatile("cp.async.bulk.prefetch.L2.global [%0], %1;" ::"l"(a), "r"(p.slab_bytes) : "memory");
+            if constexpr (sizeof(TP) == 16) {
+                asm volatile("cp.async.bulk.prefetch.L2.global [%0], %1;" ::"l"(a), "r"(p.slab_bytes) : "memory");
+            } else {
+                // bf16 slabs are 8-byte aligned: the 16-byte granules that lie inside the slab (a hint, so the ends may go unfetched)
+                const uintptr_t lo = ((uintptr_t)a + 15) & ~(uintptr_t)15, hi = ((uintptr_t)a + p.slab_bytes) & ~(uintptr_t)15;
+                if (hi > lo)
+                    asm volatile("cp.async.bulk.prefetch.L2.global [%0], %1;" ::"l"(lo), "r"((unsigned)(hi - lo)) : "memory");
+            }
         }
     }
 #endif
@@ -1322,13 +1329,23 @@ __device__ __forceinline__ int load_saved_tile_list(const Params &p, float rdt, 
 }
 #endif
 
+// One payload voxel (RGBA) of `tplate` as fp32.  The render kernels take the voxel type TP as a template parameter: float4, or
+// uint2 holding four bfloat16 (MVP_FLAG_TPLATE_BF16; R in the low half of .x).  A bfloat16 is the top half of the float with the
+// same value, so the conversion is exact and everything after the load is the fp32 kernel's arithmetic.
+__device__ __forceinline__ float4 load_voxel(const float4 *v) { return __ldg(v); }
+__device__ __forceinline__ float4 load_voxel(const uint2 *v) {
+    const uint2 u = __ldg(v);
+    return make_float4(__uint_as_float(u.x << 16), __uint_as_float(u.x & 0xffff0000u), __uint_as_float(u.y << 16),
+                       __uint_as_float(u.y & 0xffff0000u));
+}
+
 // primsampler.h:44-66 + utils.h:408-502.  T > 0: cubic slab with compile-time strides; T == 0: runtime dims.
 // Only called for valid samples (|y| < 1), for which (a) the reference's +-100 clamp is a no-op and (b) the only
 // corner that can fall outside the slab is ix+1 == TW when fx rounds to exactly TW-1, with weight exactly 0.  The
 // cell is clamped to TW-2 instead and the fractions are taken against the clamped cell: identical products in all
 // other cases (fx - ix and (ix+1) - fx are the reference's expressions), weights (1, 0) in the edge case.
-template <int T>
-__device__ __forceinline__ float4 sample_slab(const float4 *__restrict__ slab, float y0, float y1, float y2, int TD, int TH, int TW,
+template <int T, typename TP>
+__device__ __forceinline__ float4 sample_slab(const TP *__restrict__ slab, float y0, float y1, float y2, int TD, int TH, int TW,
                                               float fadescale, float fadeexp) {
     const int td = T > 0 ? T : TD, th = T > 0 ? T : TH, tw = T > 0 ? T : TW;
     const float fade = __expf(-fadescale * (__powf(fabsf(y0), fadeexp) + __powf(fabsf(y1), fadeexp) + __powf(fabsf(y2), fadeexp)));
@@ -1344,9 +1361,9 @@ __device__ __forceinline__ float4 sample_slab(const float4 *__restrict__ slab, f
     const float bz0 = fz - (float)cz, bz1 = (float)(cz + 1) - fz;
     const int sx = tw > 1 ? 1 : 0, sy = th > 1 ? tw : 0, sz = td > 1 ? th * tw : 0;
     const int base = (cz * th + cy) * tw + cx;
-    const float4 *pc = slab + base;
-    const float4 v000 = __ldg(pc), v001 = __ldg(pc + sx), v010 = __ldg(pc + sy), v011 = __ldg(pc + sy + sx);
-    const float4 v100 = __ldg(pc + sz), v101 = __ldg(pc + sz + sx), v110 = __ldg(pc + sz + sy), v111 = __ldg(pc + sz + sy + sx);
+    const TP *pc = slab + base;
+    const float4 v000 = load_voxel(pc), v001 = load_voxel(pc + sx), v010 = load_voxel(pc + sy), v011 = load_voxel(pc + sy + sx);
+    const float4 v100 = load_voxel(pc + sz), v101 = load_voxel(pc + sz + sx), v110 = load_voxel(pc + sz + sy), v111 = load_voxel(pc + sz + sy + sx);
     // (wx * wy) * wz, left-associated like the reference; corner order tnw,tne,tsw,tse,bnw,bne,bsw,bse
     const float w00 = bx1 * by1, w01 = bx0 * by1, w10 = bx1 * by0, w11 = bx0 * by0;
     float4 acc;
@@ -1391,7 +1408,8 @@ __device__ __forceinline__ CellG cell_generic(float a0, float a1, float a2, int 
 }
 
 // primsampler.h:44-66 with dowarp = true: fade from y, warp field sampled at y, payload sampled at the warped position
-__device__ __forceinline__ float4 sample_slab_warped(const float4 *__restrict__ slab, const float *__restrict__ wk, float y0, float y1,
+template <typename TP>
+__device__ __forceinline__ float4 sample_slab_warped(const TP *__restrict__ slab, const float *__restrict__ wk, float y0, float y1,
                                                      float y2, const Params &p) {
     const float fade = __expf(-p.fadescale * (__powf(fabsf(y0), p.fadeexp) + __powf(fabsf(y1), p.fadeexp) + __powf(fabsf(y2), p.fadeexp)));
     const CellG cw = cell_generic(y0, y1, y2, p.WD, p.WH, p.WW);
@@ -1408,7 +1426,7 @@ __device__ __forceinline__ float4 sample_slab_warped(const float4 *__restrict__ 
 #pragma unroll
     for (int cn = 0; cn < 8; ++cn) {
         if (ct.idx[cn] >= 0) {
-            const float4 v = __ldg(slab + ct.idx[cn]);
+            const float4 v = load_voxel(slab + ct.idx[cn]);
             acc.x = __fmaf_rn(ct.w[cn], v.x, acc.x); acc.y = __fmaf_rn(ct.w[cn], v.y, acc.y);
             acc.z = __fmaf_rn(ct.w[cn], v.z, acc.z); acc.w = __fmaf_rn(ct.w[cn], v.w, acc.w);
         }
@@ -1455,7 +1473,7 @@ struct __align__(16) FwdWarpSmem {   // per-warp shared state of the forward ker
 //    fits (almost all) with a small shared-memory footprint (more L1 for the voxel gathers) and flags the rest;
 //    the CAP == 512 variant then renders only the flagged tiles.
 // ------------------------------------------------------------------------------------------------------
-template <int T, bool kGrad, int CAP, bool kWarp>
+template <int T, bool kGrad, int CAP, bool kWarp, typename TP>
 __device__ __forceinline__ bool forward_tile(const Params &p, const int n, const int tx, const int ty, const int lane, FwdWarpSmem<CAP, kGrad> *const S) {
     // all per-warp shared state lives in one record: every address below is (one pinned per-warp base) + immediate
     int *const sk = S->k, *const siv = S->iv, *const rm = S->rm;
@@ -1494,7 +1512,7 @@ __device__ __forceinline__ bool forward_tile(const Params &p, const int n, const
     TileCtx c;
     float t, x, y, z, r1e;
     int j0;
-    if (!build_tile_list<CAP, true>(p, rdt, n, tx, ty, lane, c, sk, siv, sstage, sbar, t, x, y, z, r1e, j0)) return false;
+    if (!build_tile_list<CAP, true, TP>(p, rdt, n, tx, ty, lane, c, sk, siv, sstage, sbar, t, x, y, z, r1e, j0)) return false;
 
     const int px = tx * kTileW + (lane & 7), py = ty * kTileH + (lane >> 3);
     const size_t r = ((size_t)n * p.H + min(py, p.H - 1)) * p.W + min(px, p.W - 1);
@@ -1526,7 +1544,7 @@ __device__ __forceinline__ bool forward_tile(const Params &p, const int n, const
     // voxels per slab: a compile-time constant for the cubic 8^3 / 16^3 specialisations, so that a slab's address is a shift and an add
     // wherever the register cap makes the compiler re-derive it (it was ~30 of the 159 instructions of a batch gather)
     const size_t slabsz = T > 0 ? (size_t)(T * T * T) : (size_t)p.TD * p.TH * p.TW;
-    const float4 *tpn = reinterpret_cast<const float4 *>(p.tplate) + (size_t)(n * p.pview) * p.K * slabsz;
+    const TP *tpn = reinterpret_cast<const TP *>(p.tplate) + (size_t)(n * p.pview) * p.K * slabsz;
     const int kstart = dfs_kstart(p.K);
     {
         // pinned: under the register cap the compiler would otherwise re-materialise this base address per event
@@ -1581,7 +1599,7 @@ __device__ __forceinline__ bool forward_tile(const Params &p, const int n, const
         if (act) {
             const int kk = sk[(__float_as_int(rec.w) >> 5) & 1023];
             if (kWarp) sres = sample_slab_warped(tpn + (size_t)kk * slabsz, p.warp + ((size_t)(n * p.pview) * p.K + kk) * ((size_t)p.WD * p.WH * p.WW * 3), rec.x, rec.y, rec.z, p);
-            else sres = sample_slab<T>(tpn + (size_t)kk * slabsz, rec.x, rec.y, rec.z, p.TD, p.TH, p.TW, p.fadescale, p.fadeexp);
+            else sres = sample_slab<T, TP>(tpn + (size_t)kk * slabsz, rec.x, rec.y, rec.z, p.TD, p.TH, p.TW, p.fadescale, p.fadeexp);
         }
         __syncwarp();
         if (act) { ring[qhead + lane] = make_float4(sres.x, sres.y, sres.z, rec.w); ra[qhead + lane] = sres.w; }
@@ -1756,7 +1774,7 @@ __device__ __forceinline__ void clear_grad_slices(const Params &p, size_t g, int
     }
 }
 
-template <int T, bool kGrad, int CAP, bool kWarp>
+template <int T, bool kGrad, int CAP, bool kWarp, typename TP>
 __global__ void __launch_bounds__(kWarps * 32, (CAP < kMaxHit && !kWarp) ? (MVP_FWD_MINB * 4) / kWarps : 16 / kWarps) render_forward_kernel(const Params p) {
     __shared__ FwdWarpSmem<CAP, kGrad> s_w[kWarps];
     const int warp = threadIdx.x >> 5, lane = threadIdx.x & 31;
@@ -1767,7 +1785,7 @@ __global__ void __launch_bounds__(kWarps * 32, (CAP < kMaxHit && !kWarp) ? (MVP_
         for (int i = blockIdx.x * kWarps + warp; i < cnt; i += gridDim.x * kWarps) {
             const int id = p.heavylist[i];
             const int tx = id % p.TXn, ty = (id / p.TXn) % p.TYn, n = id / (p.TXn * p.TYn);
-            forward_tile<T, kGrad, CAP, kWarp>(p, n, tx, ty, lane, S);
+            forward_tile<T, kGrad, CAP, kWarp, TP>(p, n, tx, ty, lane, S);
             __syncwarp();
         }
     } else {
@@ -1786,7 +1804,7 @@ __global__ void __launch_bounds__(kWarps * 32, (CAP < kMaxHit && !kWarp) ? (MVP_
         long long g0_;
         asm volatile("mov.u64 %0, %%globaltimer;" : "=l"(g0_));
 #endif
-        if (!forward_tile<T, kGrad, CAP, kWarp>(p, n, tx, ty, lane, S) && lane == 0)
+        if (!forward_tile<T, kGrad, CAP, kWarp, TP>(p, n, tx, ty, lane, S) && lane == 0)
             p.heavylist[atomicAdd(p.heavycnt, 1)] = (n * p.TYn + ty) * p.TXn + tx;
 #if MVP_TILE_CLOCKS
         if (lane == 0) {
@@ -1821,13 +1839,14 @@ __device__ __forceinline__ void red_add_v4(float *addr, float a, float b, float 
 // exactly on the slab's far face: probability ~2^-24 per axis, the upper voxel is then the reference's LOWER corner and the only
 // one it sees).  Taken by those samples only; it runs after the main corner pass, when few values of the batch adjoint are live, so its
 // 12 accumulators do not add to the register peak.
-__device__ __forceinline__ float3 index_grad_general(const float4 *pc, int sx, int sy, int sz, float bx0, float bx1, float by0, float by1,
+template <typename TP>
+__device__ __forceinline__ float3 index_grad_general(const TP *pc, int sx, int sy, int sz, float bx0, float bx1, float by0, float by1,
                                                   float bz0, float bz1, float oLx, float oLy, float oLz, float A, float B, int clamp_mask) {
     const float wx_[2] = {bx1, bx0}, wy_[2] = {by1, by0}, wz_[2] = {bz1, bz0};
     float gpU[3] = {0.f, 0.f, 0.f}, gpL[3] = {0.f, 0.f, 0.f}, gaU[3] = {0.f, 0.f, 0.f}, gaL[3] = {0.f, 0.f, 0.f};
     for (int cn = 0; cn < 8; ++cn) {
         const int bx = cn & 1, byy = (cn >> 1) & 1, bz = (cn >> 2) & 1;
-        const float4 v = __ldg(pc + ((bx ? sx : 0) + (byy ? sy : 0) + (bz ? sz : 0)));
+        const float4 v = load_voxel(pc + ((bx ? sx : 0) + (byy ? sy : 0) + (bz ? sz : 0)));
         const float pr = v.x * oLx + v.y * oLy + v.z * oLz;
         const float wyz = wy_[byy] * wz_[bz], wxz = wx_[bx] * wz_[bz], wxy = wx_[bx] * wy_[byy];
         if (bx) { gpU[0] += pr * wyz; gaU[0] += v.w * wyz; } else { gpL[0] += pr * wyz; gaL[0] += v.w * wyz; }
@@ -1883,7 +1902,7 @@ __device__ __forceinline__ Prim load_rec_shared(const float4 *rec) {
     return q;
 }
 
-template <int T, int CAP, bool kWarp>
+template <int T, int CAP, bool kWarp, typename TP>
 __device__ __forceinline__ bool backward_tile(const Params &p, const int n, const int tx, const int ty, const int lane, BwdWarpSmem<CAP> *const S) {
     int *const sk = S->k, *const siv = S->iv;
     RowEntry *const sstage = S->stage;
@@ -1900,7 +1919,7 @@ __device__ __forceinline__ bool backward_tile(const Params &p, const int n, cons
     have = load_saved_tile_list<CAP>(p, rdt, n, tx, ty, lane, c, sk, siv, xb, yb, zb, j0);
     if (have == 2) return false;
 #endif
-    if (have == 0 && !build_tile_list<CAP, false>(p, rdt, n, tx, ty, lane, c, sk, siv, sstage, sbar, t0, xb, yb, zb, r1e, j0)) return false;
+    if (have == 0 && !build_tile_list<CAP, false, TP>(p, rdt, n, tx, ty, lane, c, sk, siv, sstage, sbar, t0, xb, yb, zb, r1e, j0)) return false;
     const int nl = c.nl;
     if (nl == 0) return true;
 
@@ -2071,7 +2090,7 @@ __device__ __forceinline__ bool backward_tile(const Params &p, const int n, cons
                 if (maxlen > 0 && len > 0) std::atomic_ref<long long>(g_emul_bwd_stats[3]).fetch_add(len);
 #endif
                 if (maxlen <= 0) continue;
-                const float4 *slab = reinterpret_cast<const float4 *>(p.tplate) + (pvK + k) * slabsz;
+                const TP *slab = reinterpret_cast<const TP *>(p.tplate) + (pvK + k) * slabsz;
                 float *gslab = p.g_tplate + (pvK + k) * slabsz * 4;
                 // transform-gradient accumulators of THIS lane for this slab: Gx[i][j] = sum xm_i * dL/dy_j and
                 // Gy[j] = sum dL/dy_j; grad_rot/scale/pos are linear in them (derived once per slab, before the reduction)
@@ -2188,7 +2207,7 @@ __device__ __forceinline__ bool backward_tile(const Params &p, const int n, cons
                         const float bz0 = fz - (float)cz, bz1 = (float)(cz + 1) - fz;
                         const bool ex = ix > cx, ey = iy > cy, ez = iz > cz;
                         const int base = (cz * th + cy) * tw + cx;
-                        const float4 *pc = slab + base;
+                        const TP *pc = slab + base;
                         // One pass over the 8 corners.  dL/d(sample) = (A dL.rgb, B) with A, B known only after the sample
                         // is complete, but <T_c, dL/d(sample)> = A <T_c.rgb, dL.rgb> + B T_c.a is linear in (A, B):
                         // accumulate the index-gradient sums for both parts now and combine afterwards.
@@ -2198,7 +2217,7 @@ __device__ __forceinline__ bool backward_tile(const Params &p, const int n, cons
 #pragma unroll
                         for (int cn = 0; cn < 8; ++cn) {
                             const int bx = cn & 1, byy = (cn >> 1) & 1, bz = (cn >> 2) & 1;
-                            const float4 v = __ldg(pc + ((bx ? sx : 0) + (byy ? sy : 0) + (bz ? sz : 0)));
+                            const float4 v = load_voxel(pc + ((bx ? sx : 0) + (byy ? sy : 0) + (bz ? sz : 0)));
                             const float w_ = (wx_[bx] * wy_[byy]) * wz_[bz];
                             sv.x = __fmaf_rn(w_, v.x, sv.x); sv.y = __fmaf_rn(w_, v.y, sv.y);
                             sv.z = __fmaf_rn(w_, v.z, sv.z); sv.w = __fmaf_rn(w_, v.w, sv.w);
@@ -2260,7 +2279,7 @@ __device__ __forceinline__ bool backward_tile(const Params &p, const int n, cons
 #pragma unroll
                         for (int cn = 0; cn < 8; ++cn) {
                             if (ct.idx[cn] >= 0) {
-                                const float4 v = __ldg(slab + ct.idx[cn]);
+                                const float4 v = load_voxel(slab + ct.idx[cn]);
                                 sv.x = __fmaf_rn(ct.w[cn], v.x, sv.x); sv.y = __fmaf_rn(ct.w[cn], v.y, sv.y);
                                 sv.z = __fmaf_rn(ct.w[cn], v.z, sv.z); sv.w = __fmaf_rn(ct.w[cn], v.w, sv.w);
                                 const float pr = v.x * oLx + v.y * oLy + v.z * oLz;
@@ -2381,7 +2400,7 @@ __device__ __forceinline__ bool backward_tile(const Params &p, const int n, cons
     return true;
 }
 
-template <int T, int CAP, bool kWarp>
+template <int T, int CAP, bool kWarp, typename TP>
 __global__ void __launch_bounds__(kWarps * 32, (CAP < kMaxHit && !kWarp) ? (MVP_BWD_MINB * 4) / kWarps : 12 / kWarps) render_backward_kernel(const Params p) {
     __shared__ BwdWarpSmem<CAP> s_w[kWarps];
     const int warp = threadIdx.x >> 5, lane = threadIdx.x & 31;
@@ -2391,7 +2410,7 @@ __global__ void __launch_bounds__(kWarps * 32, (CAP < kMaxHit && !kWarp) ? (MVP_
         for (int i = blockIdx.x * kWarps + warp; i < cnt; i += gridDim.x * kWarps) {
             const int id = p.heavylist[i];
             const int tx = id % p.TXn, ty = (id / p.TXn) % p.TYn, n = id / (p.TXn * p.TYn);
-            backward_tile<T, CAP, kWarp>(p, n, tx, ty, lane, S);
+            backward_tile<T, CAP, kWarp, TP>(p, n, tx, ty, lane, S);
             __syncwarp();
         }
     } else {
@@ -2404,7 +2423,7 @@ __global__ void __launch_bounds__(kWarps * 32, (CAP < kMaxHit && !kWarp) ? (MVP_
         const int tx = blockIdx.x * kBlkTX + (warp % kBlkTX), ty = blockIdx.y * kBlkTY + (warp / kBlkTX), n = blockIdx.z;
 #endif
         if (tx >= p.TXn || ty >= p.TYn) return;
-        if (!backward_tile<T, CAP, kWarp>(p, n, tx, ty, lane, S) && lane == 0)
+        if (!backward_tile<T, CAP, kWarp, TP>(p, n, tx, ty, lane, S) && lane == 0)
             p.heavylist[atomicAdd(p.heavycnt, 1)] = (n * p.TYn + ty) * p.TXn + tx;
     }
 }
@@ -2605,6 +2624,10 @@ extern "C" {
 
 int mvp_abi_version(void) { return MVP_ABI_VERSION; }
 
+int mvp_supported_flags(void) {
+    return (int)(MVP_FLAG_ACCEL_VALID | MVP_FLAG_ZERO_GRADS | MVP_FLAG_SHARED_PRIMS | MVP_FLAG_TPLATE_BF16 | MVP_FLAG_TEST_TINY_LISTS);
+}
+
 #define MVP_STR2(x) #x
 #define MVP_STR(x) MVP_STR2(x)
 const char *mvp_build_config(void) {
@@ -2626,7 +2649,7 @@ const char *mvp_error_string(int code) {
         case MVP_ERR_STEPSIZE: return "stepsize must be finite and > 0";
         case MVP_ERR_WORKSPACE: return "workspace too small or not 256-byte aligned";
         case MVP_ERR_ALGO: return "unsupported algo";
-        case MVP_ERR_ALIGN: return "misaligned buffer (tplate/rayrgba/grad_rayrgba/grad_tplate/rayaux: 16 bytes, tminmax: 8, others: 4)";
+        case MVP_ERR_ALIGN: return "misaligned buffer (tplate/rayrgba/grad_rayrgba/grad_tplate/rayaux: 16 bytes, bf16 tplate and tminmax: 8, others: 4)";
         case MVP_ERR_STRUCT: return "args->struct_size does not match this library's argument struct (ABI mismatch)";
         case MVP_ERR_CAMERA: return "camera.volradius must be finite and > 0";
         default: return code > 0 ? cudaGetErrorString((cudaError_t)code) : "unknown error";
@@ -2716,8 +2739,10 @@ int mvp_raymarch_forward(const mvp_forward_args *a, void *stream) {
     if (!(a->stepsize > 0.f) || !(a->stepsize < 3.0e38f)) return MVP_ERR_STEPSIZE;
     const Layout L = make_layout(a->shape);
     if (a->workspace_bytes < L.total || ((uintptr_t)a->workspace & 255)) return MVP_ERR_WORKSPACE;
-    // vector accesses: float4 (tplate, rayrgba), int4 (rayaux), float2 (tminmax); everything else is read as scalars
-    if (misaligned(a->tplate, 16) || misaligned(a->rayrgba, 16) || misaligned(a->rayaux, 16) || misaligned(a->tminmax, 8) ||
+    const bool bf16 = (a->flags & MVP_FLAG_TPLATE_BF16) != 0;
+    // vector accesses: float4 (tplate, rayrgba), int4 (rayaux), float2 (tminmax); everything else is read as scalars.  A bf16 tplate
+    // is read as 8-byte voxels.
+    if (misaligned(a->tplate, bf16 ? 8 : 16) || misaligned(a->rayrgba, 16) || misaligned(a->rayaux, 16) || misaligned(a->tminmax, 8) ||
         misaligned(a->raypos, 4) || misaligned(a->raydir, 4) || misaligned(a->primpos, 4) || misaligned(a->primrot, 4) ||
         misaligned(a->primscale, 4) || misaligned(a->raysat, 4) || misaligned(a->warp, 4) || misaligned(a->rayrgb_nchw, 4) ||
         misaligned(a->rayalpha_nchw, 4) || misaligned(a->order, 4) || misaligned(a->clear_grad_primpos, 16) ||
@@ -2742,6 +2767,7 @@ int mvp_raymarch_forward(const mvp_forward_args *a, void *stream) {
 #endif
     p.use_order = a->shape.N <= MVP_CTA_ORDER_MAXVIEWS;
     p.raypos = a->raypos; p.raydir = a->raydir; p.tminmax = a->tminmax; p.tplate = a->tplate;
+    if (bf16) p.slab_bytes /= 2;
     p.rayrgba = a->rayrgba; p.raysat = a->raysat; p.rayaux = reinterpret_cast<int4 *>(a->rayaux);
     p.warp = a->warp; p.WD = a->WD; p.WH = a->WH; p.WW = a->WW;
 #if MVP_CTA_ORDER
@@ -2779,22 +2805,28 @@ int mvp_raymarch_forward(const mvp_forward_args *a, void *stream) {
     }
 #endif
     const int cubic = (a->shape.TD == a->shape.TH && a->shape.TH == a->shape.TW) ? a->shape.TD : 0;
-#define MVP_LAUNCH_FWD(TT, WW_)                                                                              \
+#define MVP_LAUNCH_FWD(TT, WW_, TP_)                                                                         \
     do {                                                                                                     \
         if (a->raysat) {                                                                                     \
-            MVP_CARVE(MVP_FWD_CARVEOUT, render_forward_kernel<TT, true, kFastCapF, WW_>);                    \
-            MVP_LAUNCH_FAST(render_forward_kernel<TT, true, kFastCapF, WW_>);                                \
-            MVP_LAUNCH_HEAVY(render_forward_kernel<TT, true, kMaxHit, WW_>);                                 \
+            MVP_CARVE(MVP_FWD_CARVEOUT, render_forward_kernel<TT, true, kFastCapF, WW_, TP_>);               \
+            MVP_LAUNCH_FAST(render_forward_kernel<TT, true, kFastCapF, WW_, TP_>);                           \
+            MVP_LAUNCH_HEAVY(render_forward_kernel<TT, true, kMaxHit, WW_, TP_>);                            \
         } else {                                                                                             \
-            MVP_CARVE(MVP_FWD_CARVEOUT, render_forward_kernel<TT, false, kFastCapF, WW_>);                   \
-            MVP_LAUNCH_FAST(render_forward_kernel<TT, false, kFastCapF, WW_>);                               \
-            MVP_LAUNCH_HEAVY(render_forward_kernel<TT, false, kMaxHit, WW_>);                                \
+            MVP_CARVE(MVP_FWD_CARVEOUT, render_forward_kernel<TT, false, kFastCapF, WW_, TP_>);              \
+            MVP_LAUNCH_FAST(render_forward_kernel<TT, false, kFastCapF, WW_, TP_>);                          \
+            MVP_LAUNCH_HEAVY(render_forward_kernel<TT, false, kMaxHit, WW_, TP_>);                           \
         }                                                                                                    \
     } while (0)
-    if (a->algo == 1) MVP_LAUNCH_FWD(0, true);
-    else if (cubic == 8) MVP_LAUNCH_FWD(8, false);
-    else if (cubic == 16) MVP_LAUNCH_FWD(16, false);
-    else MVP_LAUNCH_FWD(0, false);
+#define MVP_LAUNCH_FWD_T(TP_)                                                                                \
+    do {                                                                                                     \
+        if (a->algo == 1) MVP_LAUNCH_FWD(0, true, TP_);                                                      \
+        else if (cubic == 8) MVP_LAUNCH_FWD(8, false, TP_);                                                  \
+        else if (cubic == 16) MVP_LAUNCH_FWD(16, false, TP_);                                                \
+        else MVP_LAUNCH_FWD(0, false, TP_);                                                                  \
+    } while (0)
+    if (bf16) MVP_LAUNCH_FWD_T(uint2);
+    else MVP_LAUNCH_FWD_T(float4);
+#undef MVP_LAUNCH_FWD_T
 #undef MVP_LAUNCH_FWD
     cudaError_t e = cudaGetLastError();
     return e == cudaSuccess ? MVP_OK : (int)e;
@@ -2820,7 +2852,8 @@ int mvp_raymarch_backward(const mvp_backward_args *a, void *stream) {
     if (!(a->stepsize > 0.f) || !(a->stepsize < 3.0e38f)) return MVP_ERR_STEPSIZE;
     const Layout L = make_layout(a->shape);
     if (a->workspace_bytes < L.total || ((uintptr_t)a->workspace & 255)) return MVP_ERR_WORKSPACE;
-    if (misaligned(a->tplate, 16) || misaligned(a->grad_tplate, 16) || misaligned(a->grad_rayrgba, 16) || misaligned(a->rayaux, 16) ||
+    const bool bf16 = (a->flags & MVP_FLAG_TPLATE_BF16) != 0;   // tplate only: the gradient stays fp32
+    if (misaligned(a->tplate, bf16 ? 8 : 16) || misaligned(a->grad_tplate, 16) || misaligned(a->grad_rayrgba, 16) || misaligned(a->rayaux, 16) ||
         misaligned(a->tminmax, 8) || misaligned(a->raypos, 4) || misaligned(a->raydir, 4) || misaligned(a->primpos, 4) ||
         misaligned(a->primrot, 4) || misaligned(a->primscale, 4) || misaligned(a->raysat, 4) || misaligned(a->grad_primpos, 4) ||
         misaligned(a->grad_primrot, 4) || misaligned(a->grad_primscale, 4) || misaligned(a->warp, 4) || misaligned(a->grad_warp, 4) ||
@@ -2847,6 +2880,7 @@ int mvp_raymarch_backward(const mvp_backward_args *a, void *stream) {
     p.pview = pview;
     p.raycam = camera ? reinterpret_cast<const float4 *>(ws + L.raycam) : nullptr;
     p.raypos = a->raypos; p.raydir = a->raydir; p.tminmax = a->tminmax; p.tplate = a->tplate;
+    if (bf16) p.slab_bytes /= 2;
     p.use_order = a->shape.N <= MVP_CTA_ORDER_MAXVIEWS;
     p.order = a->order; p.rankof = a->order ? reinterpret_cast<const int *>(ws + L.rankof) : nullptr;
     p.g_rgb_nchw = a->grad_rayrgb_nchw; p.g_alpha_nchw = a->grad_rayalpha_nchw;
@@ -2864,16 +2898,22 @@ int mvp_raymarch_backward(const mvp_backward_args *a, void *stream) {
         if (e0 != cudaSuccess) return (int)e0;
     }
     const int cubic = (a->shape.TD == a->shape.TH && a->shape.TH == a->shape.TW) ? a->shape.TD : 0;
-#define MVP_LAUNCH_BWD(TT, WW_)                                                                  \
+#define MVP_LAUNCH_BWD(TT, WW_, TP_)                                                             \
     do {                                                                                         \
-        MVP_CARVE(MVP_BWD_CARVEOUT, render_backward_kernel<TT, kFastCapB, WW_>);                 \
-        MVP_LAUNCH_FAST(render_backward_kernel<TT, kFastCapB, WW_>);                             \
-        MVP_LAUNCH_HEAVY(render_backward_kernel<TT, kMaxHit, WW_>);                              \
+        MVP_CARVE(MVP_BWD_CARVEOUT, render_backward_kernel<TT, kFastCapB, WW_, TP_>);            \
+        MVP_LAUNCH_FAST(render_backward_kernel<TT, kFastCapB, WW_, TP_>);                        \
+        MVP_LAUNCH_HEAVY(render_backward_kernel<TT, kMaxHit, WW_, TP_>);                         \
     } while (0)
-    if (a->algo == 1) MVP_LAUNCH_BWD(0, true);
-    else if (cubic == 8) MVP_LAUNCH_BWD(8, false);
-    else if (cubic == 16) MVP_LAUNCH_BWD(16, false);
-    else MVP_LAUNCH_BWD(0, false);
+#define MVP_LAUNCH_BWD_T(TP_)                                                                    \
+    do {                                                                                         \
+        if (a->algo == 1) MVP_LAUNCH_BWD(0, true, TP_);                                          \
+        else if (cubic == 8) MVP_LAUNCH_BWD(8, false, TP_);                                      \
+        else if (cubic == 16) MVP_LAUNCH_BWD(16, false, TP_);                                    \
+        else MVP_LAUNCH_BWD(0, false, TP_);                                                      \
+    } while (0)
+    if (bf16) MVP_LAUNCH_BWD_T(uint2);
+    else MVP_LAUNCH_BWD_T(float4);
+#undef MVP_LAUNCH_BWD_T
 #undef MVP_LAUNCH_BWD
     cudaError_t e = cudaGetLastError();
     return e == cudaSuccess ? MVP_OK : (int)e;

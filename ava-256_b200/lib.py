@@ -71,12 +71,13 @@ _sized_init(BackwardArgs)
 FLAG_ACCEL_VALID = 1
 FLAG_ZERO_GRADS = 2
 FLAG_SHARED_PRIMS = 4
+FLAG_TPLATE_BF16 = 8
 FLAG_TEST_TINY_LISTS = 0x100
 ABI_VERSION = 8
 # layout pins, equal to the static_asserts in csrc/mvp_kernels.cu (tests/test_abi.py compares)
 SIZEOF = {"Shape": 28, "Camera": 40, "ForwardArgs": 272, "BackwardArgs": 272}
 
-EXPORTS = ("mvp_abi_version", "mvp_build_config", "mvp_error_string", "mvp_workspace_bytes", "mvp_build_accel", "mvp_build_accel_camera",
+EXPORTS = ("mvp_abi_version", "mvp_supported_flags", "mvp_build_config", "mvp_error_string", "mvp_workspace_bytes", "mvp_build_accel", "mvp_build_accel_camera",
            "mvp_raymarch_forward",
            "mvp_raymarch_backward", "mvp_compute_raydirs", "mvp_forward_launch_count", "mvp_backward_launch_count",
            "mvp_composite_forward", "mvp_composite_backward", "mvp_assemble_payload_forward",
@@ -101,6 +102,8 @@ def _load():
         if not hasattr(lib, name):
             raise RuntimeError("mvpraymarch_b200: %s does not export %s" % (path, name))
     lib.mvp_abi_version.restype = ctypes.c_int
+    lib.mvp_supported_flags.restype = ctypes.c_int
+    lib.mvp_supported_flags.argtypes = []
     lib.mvp_error_string.restype = ctypes.c_char_p
     lib.mvp_build_config.restype = ctypes.c_char_p
     lib.mvp_error_string.argtypes = [ctypes.c_int]

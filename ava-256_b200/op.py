@@ -1,7 +1,8 @@
 """torch.autograd front-end of the B200 raymarcher: the host-side mirror of the reference's op
 (/root/reference/extensions/mvpraymarch/mvpraymarch.py:87-390) on top of the C-ABI in include/mvpraymarch_b200.h.
 
-Same contract as the reference: fp32 CUDA tensors, contiguous, caller-visible output rayrgba [N,H,W,4] that
+Same contract as the reference: fp32 CUDA tensors (template and primitive transforms may also be bf16, as decoders produce
+them under torch.autocast), contiguous, caller-visible output rayrgba [N,H,W,4] that
 participates in autograd with gradients for primpos, primrot, primscale, template and (algo 1) warp, None for
 everything else (mvpraymarch.py:279-292).  Differences that are deliberate:
   * kernels run on torch's current stream (the reference launches on legacy stream 0, mvpraymarch.cpp:277);
@@ -30,13 +31,19 @@ def _aligned(t, nbytes):
     return t
 
 
-def _check_f32_cuda(name, t):
+_F32 = (torch.float32,)
+# What decoders produce under torch.autocast(dtype=torch.bfloat16).  A bf16 template is read as bf16 by the kernels (C-ABI
+# MVP_FLAG_TPLATE_BF16); bf16 primitive transforms (K*60 bytes per view) are converted to fp32 here.
+_F32_BF16 = (torch.float32, torch.bfloat16)
+
+
+def _check_f32_cuda(name, t, dtypes=_F32):
     if not t.is_cuda:
         raise RuntimeError("%s must be a CUDA tensor" % name)          # mvpraymarch.cpp:102
     if not t.is_contiguous():
         raise RuntimeError("%s must be contiguous" % name)             # mvpraymarch.cpp:103
-    if t.dtype != torch.float32:
-        raise RuntimeError("%s must be float32" % name)
+    if t.dtype not in dtypes:
+        raise RuntimeError("%s must be %s" % (name, " or ".join(str(d)[len("torch."):] for d in dtypes)))
 
 
 class MVPRaymarch(Function):
@@ -73,15 +80,20 @@ class MVPRaymarch(Function):
         assert primscale.is_contiguous() and primscale.size(2) == 3
         assert template.is_contiguous() and template.dim() == 6 and template.size(-1) == 4, \
             "channels-last template [N,K,TD,TH,TW,4] required (the reference sampler is always channels-last, primsampler.h:16)"
-        for name, t in (("raypos", raypos), ("raydir", raydir), ("tminmax", tminmax), ("primpos", primpos),
-                        ("primrot", primrot), ("primscale", primscale), ("template", template)):
+        for name, t in (("raypos", raypos), ("raydir", raydir), ("tminmax", tminmax)):
             if t is not None:
                 _check_f32_cuda(name, t)
+        for name, t in (("primpos", primpos), ("primrot", primrot), ("primscale", primscale), ("template", template)):
+            _check_f32_cuda(name, t, _F32_BF16)
         if warp is not None:                                           # mvpraymarch.py:124
             assert warp.is_contiguous() and warp.dim() == 6 and warp.size(-1) == 3, \
                 "channels-last warp field [N,K,WD,WH,WW,3] required"
             _check_f32_cuda("warp", warp)
         usewarp = algo == 1                                            # algo 0 ignores a warp field, like the reference
+        # bf16 primitive transforms are rendered (and differentiated) in fp32; their gradients go back in the input dtype
+        prim_dtypes = (primpos.dtype, primrot.dtype, primscale.dtype)
+        primpos, primrot, primscale = primpos.float(), primrot.float(), primscale.float()
+        bf16 = template.dtype == torch.bfloat16
 
         if camera is not None:
             N, H, W = viewpos.size(0), int(camH), int(camW)
@@ -103,7 +115,7 @@ class MVPRaymarch(Function):
         if warp is not None:
             assert warp.shape[:2] == (NP, K), "warp disagrees with the primitives on [N,K]"
         shared = NP == 1 and N > 1
-        template, tminmax = _aligned(template, 16), _aligned(tminmax, 8)
+        template, tminmax = _aligned(template, 8 if bf16 else 16), _aligned(tminmax, 8)
         with torch.cuda.device(dev):
             wsbytes = _lib.workspace_bytes(N, H, W, K, TD, TH, TW)
             workspace = torch.empty(wsbytes, dtype=torch.uint8, device=dev)
@@ -122,7 +134,7 @@ class MVPRaymarch(Function):
             a = _lib.ForwardArgs()
             a.shape = _lib.Shape(N, H, W, K, TD, TH, TW)
             a.stepsize, a.fadescale, a.fadeexp = float(stepsize), float(options["fadescale"]), float(options["fadeexp"])
-            a.flags = _lib.FLAG_SHARED_PRIMS if shared else 0
+            a.flags = (_lib.FLAG_SHARED_PRIMS if shared else 0) | (_lib.FLAG_TPLATE_BF16 if bf16 else 0)
             a.raypos, a.raydir, a.tminmax = _ptr(raypos), _ptr(raydir), _ptr(tminmax)
             if camera is not None:
                 a.camera = _lib.Camera(_ptr(viewpos), _ptr(viewrot), _ptr(focal), _ptr(princpt), float(volradius), 0)
@@ -144,8 +156,9 @@ class MVPRaymarch(Function):
             if gradmode:
                 # The gradient buffers of the backward (mvpraymarch.py:240-246 zeros_like's them there) are made now and zero-filled
                 # by the forward's render kernel on the side (mvp_forward_args::clear_grad_*): no memset pass in the step.
-                grads = [torch.empty_like(primpos), torch.empty_like(primrot), torch.empty_like(primscale), torch.empty_like(template),
-                         torch.empty_like(warp) if usewarp else None]
+                # The template's gradient is accumulated in fp32 also for a bf16 template.
+                grads = [torch.empty_like(primpos), torch.empty_like(primrot), torch.empty_like(primscale),
+                         torch.empty_like(template, dtype=torch.float32), torch.empty_like(warp) if usewarp else None]
                 a.clear_grad_primpos, a.clear_grad_primrot, a.clear_grad_primscale = _ptr(grads[0]), _ptr(grads[1]), _ptr(grads[2])
                 a.clear_grad_tplate, a.clear_grad_warp = _ptr(grads[3]), _ptr(grads[4])
             stream = torch.cuda.current_stream(dev).cuda_stream
@@ -160,6 +173,7 @@ class MVPRaymarch(Function):
             ctx.options = options
             ctx.stepsize = float(stepsize)
             ctx.shared = shared
+            ctx.prim_dtypes = prim_dtypes
         if planes:
             return rayrgb, rayalpha
         return rayrgba
@@ -185,15 +199,18 @@ class MVPRaymarch(Function):
             grads, ctx.grads = ctx.grads, None
             fresh = grads is not None          # the forward's render kernel zero-filled them; a second backward through the
             if not fresh:                      # same graph (retain_graph) gets new ones, zero-filled by the library
-                grads = [torch.empty_like(primpos), torch.empty_like(primrot), torch.empty_like(primscale), torch.empty_like(template),
-                         torch.empty_like(warp) if usewarp else None]
+                grads = [torch.empty_like(primpos), torch.empty_like(primrot), torch.empty_like(primscale),
+                         torch.empty_like(template, dtype=torch.float32), torch.empty_like(warp) if usewarp else None]
             grad_primpos, grad_primrot, grad_primscale, grad_template, grad_warp = grads
+            del grads
             if warp is not None and not usewarp:                       # mvpraymarch.py:246 (zero when algo 0 ignores it)
                 grad_warp = torch.zeros_like(warp)
+            bf16 = template.dtype == torch.bfloat16
             a = _lib.BackwardArgs()
             a.shape = _lib.Shape(N, H, W, K, TD, TH, TW)
             a.stepsize, a.fadescale, a.fadeexp = ctx.stepsize, float(options["fadescale"]), float(options["fadeexp"])
-            a.flags = _lib.FLAG_ACCEL_VALID | (0 if fresh else _lib.FLAG_ZERO_GRADS) | (_lib.FLAG_SHARED_PRIMS if ctx.shared else 0)
+            a.flags = _lib.FLAG_ACCEL_VALID | (0 if fresh else _lib.FLAG_ZERO_GRADS) | (_lib.FLAG_SHARED_PRIMS if ctx.shared else 0) | \
+                (_lib.FLAG_TPLATE_BF16 if bf16 else 0)
             a.raypos, a.raydir, a.tminmax = _ptr(raypos), _ptr(raydir), _ptr(tminmax)
             if ctx.camera is not None:
                 viewpos, viewrot, focal, princpt, volradius = ctx.camera[:5]
@@ -214,6 +231,10 @@ class MVPRaymarch(Function):
                 a.WD, a.WH, a.WW = warp.shape[2:5]
             stream = torch.cuda.current_stream(dev).cuda_stream
             _lib.check(_lib.LIB.mvp_raymarch_backward(ctypes.byref(a), ctypes.c_void_p(stream)))
+            if bf16:                           # one round-to-nearest-even pass; the fp32 accumulator is freed here
+                grad_template = grad_template.to(torch.bfloat16)
+            pd = ctx.prim_dtypes
+            grad_primpos, grad_primrot, grad_primscale = grad_primpos.to(pd[0]), grad_primrot.to(pd[1]), grad_primscale.to(pd[2])
         return (None, None, None, None, grad_primpos, grad_primrot, grad_primscale, grad_template, grad_warp, None, None, None)
 
 
@@ -255,7 +276,7 @@ def morton_codes(primpos):
 def morton_codes_native(primpos):
     """The same codes from the library's kernel (`mvp_compute_morton`, the reference's compute_morton): the normalisation to the
     bounding box stays in torch like in the reference (mvpraymarch.py:46-50).  [N,K] int32."""
-    p = primpos.detach()
+    p = primpos.detach().float()
     cmax = p.max(dim=1, keepdim=True)[0]
     cmin = p.min(dim=1, keepdim=True)[0]
     c = ((p - cmin) / (cmax - cmin).clamp(min=1e-8)).contiguous()

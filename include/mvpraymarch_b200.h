@@ -28,7 +28,8 @@
  *
  * Conventions (same ownership model as the reference: the caller owns every buffer, outputs are written in
  * place; unlike the reference nothing is allocated inside and everything runs on the caller's stream):
- *   - all pointers are DEVICE pointers to contiguous fp32 (or int32) arrays; no torch types;
+ *   - all pointers are DEVICE pointers to contiguous fp32 (or int32) arrays; no torch types; the one exception is a bf16
+ *     tplate under MVP_FLAG_TPLATE_BF16;
  *   - `stream` is a cudaStream_t passed as void*;
  *   - return value: 0 = ok, < 0 = invalid argument (MVP_ERR_*), > 0 = a cudaError_t from the launch;
  *   - thread-safe and re-entrant: no global state.
@@ -36,7 +37,8 @@
  * Tensor layouts (SURVEY.md terminology table):
  *   raypos, raydir [N,H,W,3]   tminmax [N,H,W,2]
  *   primpos [N,K,3]  primrot [N,K,3,3] (row-major)  primscale [N,K,3] (inverse half-extents)
- *   tplate  [N,K,TD,TH,TW,4] channels-last RGBA      warp [N,K,WD,WH,WW,3] channels-last (algo 1)
+ *   tplate  [N,K,TD,TH,TW,4] channels-last RGBA, fp32 or (MVP_FLAG_TPLATE_BF16) bf16; grad_tplate is fp32 either way
+ *   warp [N,K,WD,WH,WW,3] channels-last (algo 1)
  *   rayrgba [N,H,W,4]  raysat [N,H,W,3]  rayaux [N,H,W,4] (int32, opaque; written by forward, read by backward)
  */
 #ifndef MVPRAYMARCH_B200_H_
@@ -58,7 +60,7 @@ extern "C" {
 #define MVP_ERR_WORKSPACE (-4) /* workspace too small or misaligned (256 B) */
 #define MVP_ERR_ALGO (-5)      /* algo must be 0 (no warp field) or 1 (warp field, primsampler.h:53-58) */
 #define MVP_ERR_ALIGN (-6)     /* a vector-accessed buffer is misaligned: tplate, rayrgba, grad_rayrgba, grad_tplate, rayaux
-                                * need 16 bytes, tminmax 8, everything else 4 */
+                                * need 16 bytes, a bf16 tplate (MVP_FLAG_TPLATE_BF16) and tminmax 8, everything else 4 */
 #define MVP_ERR_STRUCT (-7)    /* args->struct_size != sizeof(the struct this library was built with) */
 #define MVP_ERR_CAMERA (-8)    /* camera.volradius must be finite and > 0 */
 
@@ -74,6 +76,11 @@ typedef struct mvp_shape {
                                  * ONE that all N views share: [1,K,...] instead of [N,K,...] (SURVEY.md section 8e
                                  * "optional fast path"); gradients of all views accumulate into the one set.  Must be the
                                  * same in mvp_build_accel / forward / backward calls that share a workspace. */
+#define MVP_FLAG_TPLATE_BF16 8u  /* forward and backward: tplate holds bfloat16 [N,K,TD,TH,TW,4] ([1,K,...] with
+                                 * MVP_FLAG_SHARED_PRIMS), 8-byte aligned, instead of fp32.  Each voxel is converted to fp32 on
+                                 * load (exact), so the result is the fp32 call's on the same values.  grad_tplate and
+                                 * clear_grad_tplate stay fp32.  Must be the same in a forward and the backward that shares its
+                                 * workspace.  Check mvp_supported_flags() before setting it. */
 #define MVP_FLAG_TEST_TINY_LISTS 0x100u /* test hook: forward keeps at most 16 saved tile-list entries per view, so almost
                                  * every tile takes the backward's rebuild path */
 
@@ -162,6 +169,8 @@ typedef struct mvp_backward_args {
 } mvp_backward_args;
 
 int mvp_abi_version(void);
+/* The MVP_FLAG_* bits this library understands (a caller checks a newer flag here before it sets it). */
+int mvp_supported_flags(void);
 /* Build-time knobs of the kernels in this library, e.g. "FWD_OPAQUE=2 LIST_REUSE=1 ..." (for bench / bug reports). */
 const char *mvp_build_config(void);
 const char *mvp_error_string(int code);
